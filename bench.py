@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA, libhybvio_b200.so)
   python bench.py --impl reference ...                            the reference's own CPU path (oracle/_ref)
+  python bench.py ... --dump-outputs DIR                          also writes what the last timed step computed to DIR/*.npy
 
 A "step" is ONE stereo frame of BASELINE config 2 (EuRoC V1_02-shaped: 752x480 stereo, 150 features, 4-level pyramid,
 31x31 window, EKF state dimension 160) pushed through the whole hot path of one VIO session:
@@ -627,6 +628,41 @@ def time_kernels(sess, reps=40):
     return out
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(sess, out_dir):
+    """--dump-outputs: what the last frame of the timed device-resident loop handed its caller, as float32 / float64 arrays in
+    out_dir/<name>.npy -- optical-flow end points and statuses, the frame's pyramids, the outlier decisions of its visual updates
+    and the filter state after the augmentation. The inputs are seeded, so two builds run with the same arguments can be compared
+    file by file."""
+    sess.torch.cuda.synchronize()
+    out = {"lk_temporal_next_xy": sess.d_next.cpu().numpy()}
+    if STEREO:
+        out["lk_stereo_next_xy"] = sess.d_next2.cpu().numpy()
+    # both LK calls of a frame write the same status buffers: these are the last call's (the stereo one where there is one)
+    out["lk_status"] = sess.d_status.cpu().numpy().astype(np.float32)
+    out["lk_track_status"] = sess.d_ts.cpu().numpy().astype(np.float32)
+    for c, side in enumerate(("left", "right")[:NCAM]):
+        pyr = sess.pyr[c]                      # the loop has rotated the frame's pyramids into the "previous frame" slots
+        for lv in range(pyr.levels):
+            gray, grad = pyr.download(lv)
+            out[f"pyramid_{side}_gray_l{lv}"] = gray.astype(np.float32)
+            out[f"pyramid_{side}_grad_l{lv}"] = grad.astype(np.float32)
+    status, chi2 = sess.ekf.run_device_results(sess.nops - IMU_OPS)
+    out["ekf_outlier_status"] = status[:CHECKS].astype(np.float64)
+    out["ekf_chi2"] = chi2[:CHECKS]
+    m, P = sess.ekf.download()
+    out["ekf_mean"] = m
+    out["ekf_covariance"] = np.ascontiguousarray(P)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_MAX_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def ctypes_slice(arr, start, count):
     import ctypes
     return ctypes.cast(ctypes.byref(arr, start * ctypes.sizeof(arr._type_)), ctypes.POINTER(arr._type_))
@@ -788,9 +824,11 @@ def run_ours(args):
         clocks = sampler.stop() if sampler else None
         barrier()
         ms_dev = aggregate_ms(ms_local, sess.dev, world)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(sess, args.dump_outputs)
         if args.step_only:
             if rank == 0:
-                print(json.dumps({"metric": METRIC(), "value": round(frames_per_second(world * nsess, args.steps, ms_dev), 2), "steps": args.steps,
+                emit(json.dumps({"metric": METRIC(), "value": round(frames_per_second(world * nsess, args.steps, ms_dev), 2), "steps": args.steps,
                                   "warmup": args.warmup, "gpu_launches": launches, "note": "--step-only: device-resident loop only, no e2e / kernel rows"}))
             return
         e2e_steps = max(3, min(args.steps, args.e2e_steps))
@@ -1138,8 +1176,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS), help="BASELINE.json config: 2 (default, the headline), 4 (512x512, 200 features, N=62), 1 (mono)")
     ap.add_argument("--step-only", action="store_true", help="only the device-resident timed loop (for `ncu` launch lists of the step: profiles/README.md)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (end points, statuses, "
+                                                           "pyramids, outlier decisions, filter state) as DIR/<name>.npy (CUDA arm)")
     ap.add_argument("--selftest-dist", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm (--impl ours)")
     args.warmup = max(3, args.warmup)
     set_config(args.config)
     if args.selftest_dist:
